@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: rasterizer fwd+bwd frames/s @ 1 M Gaussians, 1200x680 (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0). See DESIGN.md "Measurement" for what every field means.
 * value      : frames/s with the Gaussian map, camera and upstream gradients resident in HBM (device events).
@@ -41,7 +41,11 @@ def parse():
     ap.add_argument("--gaussians", type=int, default=1_000_000)
     ap.add_argument("--camera", default="replica")
     ap.add_argument("--no-extras", action="store_true", help="skip cpu_baseline / reference-CUDA / ICP / Adam side measurements")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def workload_name(P, cam):
@@ -144,6 +148,51 @@ def run_reference_arm(args):
         "gpu_launches": 0,
     }
     print(json.dumps(line), flush=True)
+
+
+# --------------------------------------------------------------------------- outputs of the timed path
+DUMP_MAPS = ("color", "depth", "hit_color", "hit_depth", "hit_color_weight", "hit_depth_weight", "T_map")
+DUMP_GRADS = (("means3D", "xyz"), ("shs", "shs"), ("opacities", "opacity"), ("scales", "scales"), ("rotations", "rotations"))
+DUMP_PIXELS = 1_000_000     # frames above this (1920x1080) keep a seeded pixel sample
+DUMP_ROWS = 1 << 15         # per-Gaussian outputs keep a seeded sample of the Gaussians
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(path, out, grads):
+    """Writes the rasterizer outputs `out` and the per-Gaussian gradients `grads` of one step as DIR/<name>.npy: floats
+    as float32, index maps and radii as float64 (exact). Pixel maps keep shape (C, H, W), or (C, n) at the pixels of
+    pixel_index.npy when the frame has more than DUMP_PIXELS pixels; radii.npy and grad_<name>.npy hold the Gaussians
+    of gaussian_index.npy. Both samples are seeded, so the same arguments give the same files in any build."""
+    import torch
+
+    def pick(n, k, seed):
+        if n <= k:
+            return None
+        return np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
+
+    H, W = out[0].shape[-2:]
+    P = out[7].shape[0]
+    px, rows = pick(H * W, DUMP_PIXELS, 1), pick(P, DUMP_ROWS, 2)
+    rows = np.arange(P) if rows is None else rows
+    dev_rows = torch.from_numpy(rows).to(out[7].device)
+    arrays = {}
+    for name, t in zip(DUMP_MAPS, out):
+        t = t.detach()
+        arrays[name] = t if px is None else t.reshape(t.shape[0], -1)[:, torch.from_numpy(px).to(t.device)]
+    arrays["radii"] = out[7].detach()[dev_rows]
+    for name, g in grads.items():
+        arrays["grad_" + name] = g.detach()[dev_rows]
+    if px is not None:
+        arrays["pixel_index"] = torch.from_numpy(px)
+    arrays["gaussian_index"] = torch.from_numpy(rows)
+    host = {k: v.cpu().numpy() for k, v in arrays.items()}
+    host = {k: v.astype(np.float64 if v.dtype.kind in "iub" else np.float32, copy=False) for k, v in host.items()}
+    total = sum(v.nbytes for v in host.values())
+    if total > DUMP_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed {DUMP_BYTES}")
+    os.makedirs(path, exist_ok=True)
+    for k, v in host.items():
+        np.save(os.path.join(path, k + ".npy"), v)
 
 
 # --------------------------------------------------------------------------- our arm
@@ -257,13 +306,19 @@ def main():
     marks = [torch.cuda.Event(enable_timing=True) for _ in range(args.steps)]  # per-step spread (SURVEY 8(d): median, p10/p90)
     e0.record()
     for k in range(args.steps):
-        step()
+        if k == args.steps - 1:
+            out = step()  # only the last step's outputs are held on to (--dump-outputs)
+        else:
+            step()
         marks[k].record()
     drain()  # the last two all-reduces end inside the timed region
     e1.record()
     barrier()
     _lib.profile_enable(False)
     prof = _lib.profile_read(reset=True)
+    if args.dump_outputs and rank == 0:  # before anything else renders or steps the map
+        grads = flats[(tick["k"] - 1) & 1].views if flats else {n: leaves[k].grad for n, k in DUMP_GRADS}
+        dump_outputs(args.dump_outputs, out, grads)
     ms_total = e0.elapsed_time(e1)
     tm = torch.tensor([ms_total], device=dev, dtype=torch.float64)
     if world > 1:

@@ -3,6 +3,7 @@ extension has been built into oracle/_ref/) the reference's own CUDA rasterizer.
 from __future__ import annotations
 
 import glob
+import hashlib
 import importlib.util
 import os
 
@@ -111,6 +112,113 @@ def run_ref_cuda(cam, g, device, tile_mask=None, grads=None, **over):
                             rotations=grot.cpu().numpy(), means2D=g2d.cpu().numpy(), colors=gcol.cpu().numpy(),
                             cov3D=gcov.cpu().numpy())
     return res
+
+
+# ---------------------------------------------------------------- stored samples of the reference's CUDA extensions
+# tests/golden/make_reference_cuda_golden.py runs the reference's own extensions (oracle/_ref) on the inputs below. Their
+# full outputs at these sizes are tens of MB, so the fixtures keep a seeded sample of each output plus the whole-array
+# figures the assertions need (maxima, run-to-run jitter, a digest where the comparison is exact); the tests draw the
+# same samples from the same seeds.
+def sample_indices(n, k, seed):
+    """`k` distinct indices of range(n), ascending (all of range(n) when k >= n)."""
+    if k >= n:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
+
+
+def digest(a):
+    """SHA-256 of an array's dtype, shape and values (-0.0 hashed as 0.0): exact equality with an array that is not stored."""
+    a = np.ascontiguousarray(a)
+    if a.dtype.kind == "f":
+        a = a + a.dtype.type(0)
+    return hashlib.sha256(f"{a.dtype.str}{a.shape}".encode() + a.tobytes()).hexdigest()
+
+
+# (camera, Gaussians, tile-mask keep fraction). The last four are the timed configurations: BASELINE.json configs[1]
+# (~300 k @1200x680), the headline scene of bench.py (1 M @1200x680: its longest tile list exceeds the 4096-key
+# on-chip sort, i.e. the chunked-merge path), the same with a 50 % tile mask, and configs[2] (1 M @1920x1080).
+LIVE_CASES = [("tum", 10_000, None), ("replica", 60_000, None), ("replica", 300_000, None), ("replica", 1_000_000, None),
+              ("replica", 1_000_000, 0.5), ("hd", 1_000_000, None)]
+LIVE_PIXELS = 2048          # sampled pixels per case: the 5e-4 outlier allowance still admits one
+LIVE_ROWS = 128             # sampled visible Gaussians per case, besides the 8 largest gradient rows of each tensor
+PIXEL_MAPS = ("color", "depth", "hit_color", "hit_depth", "hit_color_weight", "hit_depth_weight", "T_map")
+GRADS = ("means3D", "shs", "opacities", "scales", "rotations")
+
+
+def live_case(camname, P, keep):
+    """Scene, tile mask, upstream gradients and the fixture key of one LIVE_CASES entry."""
+    from rtg_slam_b200 import scene
+    cam = scene.make_camera(camname)
+    g = scene.surfel_room(P, seed=2024)
+    mask = None if keep is None else scene.random_tile_mask(cam, keep, seed=11)
+    grads = scene.upstream_grads(cam, seed=5)
+    return cam, g, mask, grads, f"{camname}_{P}_{keep}"
+
+
+def live_pixels(cam):
+    return sample_indices(cam.height * cam.width, LIVE_PIXELS, seed=cam.height * cam.width)
+
+
+def pixel_sample(maps, px):
+    """The pixel maps of a render at the flat pixel indices `px`, shaped (C, 1, len(px)) for compare_outputs."""
+    return {k: maps[k].reshape(maps[k].shape[0], 1, -1)[..., px] for k in PIXEL_MAPS}
+
+
+# BASELINE configs[3], second half: 10 mapping iterations (render -> colour + depth L1 -> backward -> Adam) on this map.
+# Colours / rotations / opacity take the lrs of configs/base.yaml:82-86; position and scale are optimised here in their
+# activated form (the mapper steps log-scales), so their lrs are scaled down to keep the 10 steps a descent.
+OPT_LOOP_LRS = dict(xyz=1e-4, shs=5e-4, opacity=0.0, scales=1e-4, rotations=1e-3)
+OPT_LOOP_ITERS = 10
+OPT_LOOP_SAMPLE = 8192      # sampled elements of each optimised parameter tensor
+
+
+def optimize_loop_case(device):
+    """(camera, rasterization settings, initial parameters, target colour (H,W,3), target depth (H,W)): the target frame is
+    this library's render of the same map with perturbed colours and positions."""
+    from rtg_slam_b200 import scene
+    from rtg_slam_b200.rasterizer import GaussianRasterizer
+    cam = scene.make_camera("tum")
+    g = scene.surfel_room(20_000, seed=31)
+    rs = make_settings(cam, device)
+    t = to_torch(g, device)
+    with torch.no_grad():
+        tgt = GaussianRasterizer(rs)(means3D=t["xyz"] + 0.002, opacities=t["opacity"], shs=t["shs"] * 0.9, scales=t["scales"],
+                                     rotations=t["rotations"])
+    return cam, rs, t, tgt[0].permute(1, 2, 0).contiguous(), tgt[1][0].contiguous()
+
+
+def optimize_loop_sample(k, t):
+    return sample_indices(t[k].numel(), OPT_LOOP_SAMPLE, seed=sum(map(ord, k)))
+
+
+# GaussianPointCloud.update_geometry's distCUDA2 on a 300 k-point surface map (test_mapsurgery_gpu.py)
+KNN_ROWS = 8192
+
+
+# Mapping's accumulate_gaussian_error (cuda_utils): (H, W, P) cases of test_mapstats_gpu.py
+ACCUMULATE_CASES = [(680, 1200, 200_000), (77, 45, 300), (16, 16, 1)]
+ACCUMULATE_ROWS = 4096
+ACCUMULATE_THRESHOLDS = (0.3, 0.05, 0.5)
+
+
+def accumulate_inputs(H, W, P, seed):
+    """Colour / depth / normal error maps and colour / depth index maps, (H, W, 1) each."""
+    rng = np.random.default_rng(seed)
+    ce = rng.uniform(0, 1, (H, W, 1)).astype(np.float32) ** 2
+    de = rng.uniform(0, 0.2, (H, W, 1)).astype(np.float32)
+    ne = rng.uniform(0, 1, (H, W, 1)).astype(np.float32)
+    de[rng.uniform(size=(H, W, 1)) < 0.2] = 0
+    ci = rng.integers(-1, P, (H, W, 1)).astype(np.int32)     # -1 = no Gaussian
+    di = rng.integers(-1, P, (H, W, 1)).astype(np.int32)
+    hot = rng.uniform(size=(H, W, 1)) < 0.3                    # many pixels on few Gaussians: contended atomics
+    ci[hot] = rng.integers(0, min(P, 17), int(hot.sum()))
+    ci[0, 0, 0], di[0, 0, 0] = P, P + 5                        # out of range: skipped
+    return ce, de, ne, ci, di
+
+
+def accumulate_exact(k, check_max):
+    """Maxima and integer counts are order-independent (bit-exact); fp32 atomic sums are not."""
+    return check_max or k == 3
 
 
 # ---------------------------------------------------------------- comparison

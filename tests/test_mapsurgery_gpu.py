@@ -1,8 +1,6 @@
 """GPU parity of the map-surgery and nearest-neighbour entry points (SURVEY 8(f) #4) through the C ABI: against the
-numpy oracle (brute force), against scipy's k-d tree at a size the brute force cannot reach, and -- when
-oracle/_ref/simple_knn holds it (built unmodified by oracle/build_ref.py) -- against the reference's own distCUDA2."""
-import glob
-import importlib.util
+numpy oracle (brute force), against scipy's k-d tree at a size the brute force cannot reach, and against the reference's
+own distCUDA2 (simple-knn built unmodified by oracle/build_ref.py; tests/golden/knn_dist_cuda2.npz holds its outputs)."""
 import os
 
 import numpy as np
@@ -14,16 +12,6 @@ from oracle import knn_oracle as ko
 from rtg_slam_b200 import mapsurgery, scene
 
 pytestmark = pytest.mark.gpu
-
-
-def _ref_simple_knn():
-    so = glob.glob(os.path.join(helpers.ROOT, "oracle", "_ref", "simple_knn", "_C_simple_knn*.so"))
-    if not so:
-        return None
-    spec = importlib.util.spec_from_file_location("_C_simple_knn", so[0])
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
 
 
 def _surface_points(n, seed):
@@ -87,12 +75,12 @@ def test_dist_cuda2_large_against_kdtree_and_reference(cuda_device):
     dd, _ = cKDTree(pts.astype(np.float64)).query(pts.astype(np.float64), k=4)
     want = (dd[:, 1:] ** 2).mean(1)
     assert np.allclose(mean.cpu().numpy(), want, rtol=1e-4, atol=1e-10)
-    ref = _ref_simple_knn()
-    if ref is not None:  # the reference's own distCUDA2 on the same device
-        rmean, ridx = ref.distCUDA2(t)
-        assert np.allclose(mean.cpu().numpy(), rmean.cpu().numpy(), rtol=2e-6, atol=1e-12)
-        a, b = np.sort(idx.cpu().numpy(), 1), np.sort(ridx.cpu().numpy(), 1)
-        assert (a != b).any(1).mean() < 0.05  # indices differ only among equidistant neighbours (the planted duplicates)
+    # the reference's own distCUDA2 on the same points, at a seeded sample of them (make_reference_cuda_golden.py)
+    gold = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "knn_dist_cuda2.npz"))
+    rows = helpers.sample_indices(n, helpers.KNN_ROWS, seed=n)
+    assert np.allclose(mean.cpu().numpy()[rows], gold["mean"], rtol=2e-6, atol=1e-12)
+    a = np.sort(idx.cpu().numpy(), 1)[rows]
+    assert (a != gold["idx_sorted"]).any(1).mean() < 0.05  # indices differ only among equidistant neighbours (the planted duplicates)
 
 
 def test_update_geometry_expression_on_our_knn(cuda_device):

@@ -1,6 +1,6 @@
 """GPU parity tests of the rasterizer (through the public operator API -> ctypes -> C ABI -> sm_100a kernels)
-against the CPU oracle, the committed golden outputs of the reference's CUDA code, and -- when oracle/_ref holds
-the reference extension -- the reference itself on the same device.
+against the CPU oracle and the committed golden outputs of the reference's CUDA code (small scenes in full, the timed
+configurations and an optimisation loop as seeded samples).
 
 Tolerances (SURVEY.md section 8(c)): float maps L_inf < 1e-4; index maps exact outside pixels whose deciding
 alpha / T is within 1e-4 (relative) of a threshold (flagged by the oracle); per-tensor gradient
@@ -62,29 +62,23 @@ def test_matches_reference_cuda_golden(cuda_device, name):
         assert helpers.rel_err(ours["grads"][k], gold["grad_" + k]) < tol, k
 
 
-# (camera, Gaussians, tile-mask keep fraction). The last four are the timed configurations: BASELINE.json configs[1]
-# (~300 k @1200x680), the headline scene of bench.py (1 M @1200x680: its longest tile list exceeds the 4096-key
-# on-chip sort, i.e. the chunked-merge path), the same with a 50 % tile mask, and configs[2] (1 M @1920x1080).
-LIVE_CASES = [("tum", 10_000, None), ("replica", 60_000, None), ("replica", 300_000, None), ("replica", 1_000_000, None),
-              ("replica", 1_000_000, 0.5), ("hd", 1_000_000, None)]
-
-
-@pytest.mark.parametrize("camname,P,keep", LIVE_CASES)
+@pytest.mark.parametrize("camname,P,keep", helpers.LIVE_CASES)
 def test_matches_live_reference_cuda(cuda_device, camname, P, keep):
-    if helpers.ref_cuda_module() is None:
-        pytest.skip("oracle/_ref not built")
-    cam = scene.make_camera(camname)
-    g = scene.surfel_room(P, seed=2024)
-    mask = None if keep is None else scene.random_tile_mask(cam, keep, seed=11)
-    grads = scene.upstream_grads(cam, seed=5)
+    """The timed configurations against the reference's own CUDA rasterizer, as stored by make_reference_cuda_golden.py:
+    pixel maps at a seeded pixel sample, gradients at the sampled rows over the reference's max |g| of the whole tensor,
+    radii exactly (digest)."""
+    gold = np.load(os.path.join(GOLD, "live_raster_reference.npz"))
+    cam, g, mask, grads, c = helpers.live_case(camname, P, keep)
     ours = helpers.run_ours(cam, g, cuda_device, tile_mask=mask, grads=grads)
-    ref = helpers.run_ref_cuda(cam, g, cuda_device, tile_mask=mask, grads=grads)
-    ref2 = helpers.run_ref_cuda(cam, g, cuda_device, tile_mask=mask, grads=grads)
-    st = helpers.compare_outputs(ours, ref, tol=1e-4, max_bad_frac=5e-4, label=f"{camname}/{P}/{keep}")
-    assert st["radii_mismatch"] == 0
+    rows = gold[f"{c}_rows"]
+    a = dict(helpers.pixel_sample(ours, helpers.live_pixels(cam)), radii=ours["radii"][rows])
+    b = dict({k: gold[f"{c}_{k}"][:, None] for k in helpers.PIXEL_MAPS}, radii=gold[f"{c}_radii"])
+    st = helpers.compare_outputs(a, b, tol=1e-4, max_bad_frac=5e-4, label=f"{camname}/{P}/{keep}")
+    assert st["radii_mismatch"] == 0 and helpers.digest(ours["radii"].astype(np.int32)) == str(gold[f"{c}_radii_digest"])
     for k in GRADS:
-        jitter = helpers.rel_err(ref2["grads"][k], ref["grads"][k])
-        assert helpers.rel_err(ours["grads"][k], ref["grads"][k]) < max(1e-3, 10 * jitter), (k, jitter)
+        jitter = float(gold[f"{c}_jitter_{k}"])
+        err = np.abs(ours["grads"][k][rows].astype(np.float64) - gold[f"{c}_grad_{k}"]).max() / (float(gold[f"{c}_gradmax_{k}"]) + 1e-12)
+        assert err < max(1e-3, 10 * jitter), (k, err, jitter)
 
 
 def test_sh_degrees_and_background(cuda_device):
@@ -434,95 +428,46 @@ def test_optimize_loop_tracks_reference_rasterizer_with_torch_adam(cuda_device):
     torch.optim.Adam (eps = 1e-15, lrs of configs/base.yaml:82-86, as Mapping.local_optimize sets it up). The loss must
     follow the same trajectory and the parameters must agree; with eps = 1e-15 Adam's update is sign(g) * lr for a
     gradient of any magnitude, so the handful of elements whose gradient is numerically zero may step the other way
-    (atomic-order noise of the reference itself): they are bounded in number and by 2 * lr * iterations."""
-    mod = helpers.ref_cuda_module()
-    if mod is None:
-        pytest.skip("oracle/_ref not built")
+    (atomic-order noise of the reference itself): they are bounded in number and by 2 * lr * iterations. The reference's
+    side (losses, the parameters after the loop at a seeded element sample, max |p|, max |p - p0|, its run-to-run spread)
+    is stored by make_reference_cuda_golden.py."""
     from rtg_slam_b200.loss import l1_color_depth_loss
     from rtg_slam_b200.optim import FusedAdam
     from rtg_slam_b200.rasterizer import GaussianRasterizer
-    dev = cuda_device
-    cam = scene.make_camera("tum")
-    P = 20_000
-    g = scene.surfel_room(P, seed=31)
-    rs = helpers.make_settings(cam, dev)
-    t = helpers.to_torch(g, dev)
-    H, W = cam.height, cam.width
-    with torch.no_grad():  # target frame: the same map with perturbed colours / positions
-        tgt = GaussianRasterizer(rs)(means3D=t["xyz"] + 0.002, opacities=t["opacity"], shs=t["shs"] * 0.9, scales=t["scales"],
-                                     rotations=t["rotations"])
-    gt_color, gt_depth = tgt[0].permute(1, 2, 0).contiguous(), tgt[1][0].contiguous()
-    names = ("xyz", "shs", "opacity", "scales", "rotations")
-    # lrs of configs/base.yaml:82-86 for the colours / rotations / opacity; position and scale are optimised here in their
-    # activated form (the mapper steps log-scales), so their lrs are scaled down to keep the 10 steps a descent
-    lrs = dict(xyz=1e-4, shs=5e-4, opacity=0.0, scales=1e-4, rotations=1e-3)
-    iters = 10
+    gold = np.load(os.path.join(GOLD, "optimize_loop_reference.npz"))
+    cam, rs, t, gt_color, gt_depth = helpers.optimize_loop_case(cuda_device)
+    lrs, iters = helpers.OPT_LOOP_LRS, helpers.OPT_LOOP_ITERS
+    names = tuple(lrs)
 
-    class RefRaster(torch.autograd.Function):  # the reference's python shim, reduced to what the loop needs
-        @staticmethod
-        def forward(ctx, xyz, shs, opacity, scales, rotations):
-            e = torch.Tensor([])
-            th, tw = cam.tile_grid
-            tm = torch.ones((th, tw), dtype=torch.int32, device=dev)
-            st = helpers.DEFAULT_SETTINGS
-            out = mod.rasterize_gaussians(rs.bg, xyz, e, opacity, scales, rotations, st["scale_modifier"], e, rs.viewmatrix, rs.projmatrix, tm,
-                                          cam.tanfovx, cam.tanfovy, H, W, cam.cx, cam.cy, shs, st["sh_degree"], st["color_sigma"], rs.campos,
-                                          st["opaque_threshold"], st["depth_threshold"], st["normal_threshold"], st["T_threshold"], False, False)
-            ctx.state = out
-            ctx.save_for_backward(xyz, shs, scales, rotations)
-            return out[2], out[3], out[5]
-
-        @staticmethod
-        def backward(ctx, gc, gd, _):
-            (num_rendered, num_tile, color, depth, hit_color, hit_depth, hcw, hdw, T_map, radii, geomB, binB, imgB, tile_indices) = ctx.state
-            xyz, shs, scales, rotations = ctx.saved_tensors
-            e = torch.Tensor([])
-            st = helpers.DEFAULT_SETTINGS
-            (g2d, gcol, gop, gm3, gcov, gsh, gsc, grot) = mod.rasterize_gaussians_backward(
-                tile_indices, num_tile, rs.bg, xyz, radii, e, scales, rotations, st["scale_modifier"], e, rs.viewmatrix, rs.projmatrix,
-                cam.tanfovx, cam.tanfovy, cam.cx, cam.cy, st["depth_threshold"], st["normal_threshold"], gc.contiguous(), gd.contiguous(), shs,
-                st["sh_degree"], rs.campos, geomB, num_rendered, binB, imgB, hit_depth, False)
-            return gm3, gsh, gop, gsc, grot
-
-    def run(ours):
+    def run():
         p = {k: t[k].clone().requires_grad_(True) for k in names}
-        groups = [{"params": [p[k]], "lr": lrs[k]} for k in names]
-        opt = (FusedAdam if ours else torch.optim.Adam)(groups, lr=0.0, eps=1e-15)
+        opt = FusedAdam([{"params": [p[k]], "lr": lrs[k]} for k in names], lr=0.0, eps=1e-15)
         losses = []
         for _ in range(iters):
             opt.zero_grad(set_to_none=True)
-            if ours:
-                out = GaussianRasterizer(rs)(means3D=p["xyz"], opacities=p["opacity"], shs=p["shs"], scales=p["scales"], rotations=p["rotations"])
-                loss, _ = l1_color_depth_loss({"render": out[0], "depth": out[1], "depth_index_map": out[3]}, gt_color, gt_depth,
-                                              color_weight=0.8, depth_weight=1.0, depth_error_max=0.1)
-            else:
-                color, depth, hit_depth = RefRaster.apply(p["xyz"], p["shs"], p["opacity"], p["scales"], p["rotations"])
-                image, d, di = color.permute(1, 2, 0), depth.permute(1, 2, 0), hit_depth.permute(1, 2, 0)
-                color_loss = torch.abs(image - gt_color).mean()
-                err = d - gt_depth[..., None]
-                valid = (di != -1).squeeze() & (gt_depth > 0) & (err < 0.1).squeeze()
-                loss = 1.0 * torch.abs(err[valid]).mean() + 0.8 * color_loss
+            out = GaussianRasterizer(rs)(means3D=p["xyz"], opacities=p["opacity"], shs=p["shs"], scales=p["scales"], rotations=p["rotations"])
+            loss, _ = l1_color_depth_loss({"render": out[0], "depth": out[1], "depth_index_map": out[3]}, gt_color, gt_depth,
+                                          color_weight=0.8, depth_weight=1.0, depth_error_max=0.1)
             loss.backward()
             opt.step()
             losses.append(float(loss.detach()))
         return losses, {k: v.detach().clone() for k, v in p.items()}
 
-    la, pa = run(True)
-    lb, pb = run(False)
-    lc, pc = run(False)  # the reference loop a second time: its own run-to-run spread (atomic order) is the yardstick
+    la, pa = run()
+    lb = [float(x) for x in gold["losses"]]
     assert lb[-1] < lb[0], ("the loop must make progress", lb)
     for a, b in zip(la, lb):
         assert abs(a - b) < 2e-4 * abs(b), (la, lb)
     report = {}
     for k in names:
-        scale = float(pb[k].abs().max())
-        moved = float((pb[k] - t[k]).abs().max())
+        scale = float(gold[f"{k}_scale"])
+        moved = float(gold[f"{k}_moved"])
         if lrs[k] == 0.0:
-            assert torch.equal(pa[k], pb[k]) and moved == 0.0  # opacity_lr is 0 in every shipped config
+            assert torch.equal(pa[k], t[k]) and moved == 0.0  # opacity_lr is 0 in every shipped config
             continue
-        d_ours, d_self = (pa[k] - pb[k]).abs(), (pc[k] - pb[k]).abs()
-        off_ours = float((d_ours > 1e-5 * scale).float().mean())
-        off_self = float((d_self > 1e-5 * scale).float().mean())
+        d_ours = np.abs(pa[k].reshape(-1).cpu().numpy()[helpers.optimize_loop_sample(k, t)] - gold[f"{k}_sample"])
+        off_ours = float((d_ours > 1e-5 * scale).mean())
+        off_self = float(gold[f"{k}_off_self"])
         report[k] = (off_ours, off_self)
         assert moved > 0
         assert float(d_ours.max()) <= 2.0 * lrs[k] * iters + 1e-7, k  # a flipped element is at most 2*lr per step away
